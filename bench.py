@@ -42,6 +42,7 @@ import os
 import statistics
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -259,6 +260,38 @@ def cpu_baseline(spec, hf_weights, vocab, rows, threads: int, budget_s: float = 
                       "oracle/model_ref.py (torch CPU fp32 GEMM on bf16-valued weights); the "
                       "reference repo has no local implementation of this path",
             "output_tokens_per_s": n_out / dt}, texts, min_margins
+
+
+DUMP_LIMIT = 64 << 20   # bytes, both --dump-outputs files together
+
+
+def dump_width(vocab, max_new_tokens: int) -> int:
+    """Longest result string, in code points, a job can return: at most `max_new_tokens`
+    tokens (forced tokens included), decoded with errors='replace', which never yields
+    more code points than bytes."""
+    return max_new_tokens * max(len(b) for b in vocab.token_bytes)
+
+
+def dump_outputs(dirname: str, outputs, width: int, limit: int = DUMP_LIMIT):
+    """--dump-outputs: the result column of the last timed step, as the caller receives it.
+    `inference_result.npy` holds row r's Unicode code points as float32 values (exact up to
+    U+10FFFF), padded with -1 to `width` (dump_width); `row_index.npy` (float64) gives the
+    frame row of each line.  If all rows would not fit in `limit` bytes, a fixed seeded
+    sample of rows is written instead.  Width and sample follow from the row count and the
+    arguments only, so two builds run with the same arguments write arrays of one shape."""
+    import numpy as np
+    n = len(outputs)
+    keep = min(n, (limit - 4096) // (4 * width + 8))     # 4096: room for the two .npy headers
+    idx = np.arange(n) if keep == n else \
+        np.sort(np.random.RandomState(0).choice(n, keep, replace=False))
+    arr = np.full((len(idx), width), -1.0, dtype=np.float32)
+    for r, i in enumerate(idx):
+        cp = np.frombuffer(outputs[i].encode("utf-32-le"), dtype="<u4")
+        arr[r, :len(cp)] = cp
+    os.makedirs(dirname, exist_ok=True)
+    np.save(os.path.join(dirname, "inference_result.npy"), arr)
+    np.save(os.path.join(dirname, "row_index.npy"), idx.astype(np.float64))
+    log(f"dumped {len(idx)}/{n} result rows to {dirname}")
 
 
 def plumbing_cost(model, rows, outputs):
@@ -543,7 +576,15 @@ def main():
     ap.add_argument("--kv-pages", type=int, default=None,
                     help="KV pool size in pages (default: 80%% of free memory); small pools keep "
                          "ncu's save/restore cheap")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last step's result column to DIR as "
+                         ".npy (code points as float32, at most 64 MB; a seeded row sample if "
+                         "larger)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the GPU arm computed (--impl ours)")
     global WORKLOAD
     WORKLOAD = args.workload
     divert_stdout()
@@ -583,7 +624,9 @@ def main():
     vocab = VB.build_vocab(spec.family, spec.vocab_size, seed=0)
     eng = LocalEngine(spec, weights, vocab, device=dev, max_slots=args.max_slots,
                       max_prefill_tokens=args.max_prefill_tokens, kv_pages=args.kv_pages)
-    client = Sutro(verbose=False, cache_dir="/tmp/sb200-bench-cache")
+    # results cache private to this run: a fixed path under /tmp may belong to another user
+    cache = tempfile.TemporaryDirectory(prefix="sb200-bench-cache-")
+    client = Sutro(verbose=False, cache_dir=cache.name)
     client.register_engine(args.model, eng)
     setup_s = time.perf_counter() - t0
     log(f"engine ready in {setup_s:.1f}s (kv_pages={eng.kv_pages})")
@@ -652,6 +695,9 @@ def main():
         launches = sum(launches_of(s) for s in stats)
         total_rows = args.rows * args.steps
         outputs = list(frames[-1]["inference_result"])
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs,
+                         dump_width(vocab, gen_kwargs()["max_new_tokens"]))
         if WORKLOAD == "sentiment":
             ok = all(json.loads(o)["sentiment"] in ("positive", "neutral", "negative")
                      for i in range(args.warmup, n_frames)

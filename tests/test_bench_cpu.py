@@ -13,8 +13,39 @@ def test_bench_imports_and_prints_usage():
                          capture_output=True, text=True, timeout=300)
     assert out.returncode == 0, out.stderr[-2000:]
     for flag in ("--gpus", "--steps", "--warmup", "--impl", "--rows", "--workload",
-                 "--no-secondary"):
+                 "--no-secondary", "--dump-outputs"):
         assert flag in out.stdout
+
+
+def test_dump_outputs_round_trip_and_sample(tmp_path):
+    sys.path.insert(0, ROOT)
+    import numpy as np
+    import bench
+    from sutro_b200 import vocab as VB
+    outs = ['{"sentiment":"positive"}', '{"sentiment":"neutral"}', "café 🙂 \ufffd", ""] * 50
+
+    def read(d):
+        a, idx = np.load(d / "inference_result.npy"), np.load(d / "row_index.npy")
+        assert a.dtype == np.float32 and idx.dtype == np.float64
+        rows = ["".join(chr(int(x)) for x in r if x >= 0) for r in a]
+        return a.shape, rows, idx.astype(int).tolist()
+
+    bench.dump_outputs(str(tmp_path / "all"), outs, width=30)
+    shape, rows, idx = read(tmp_path / "all")
+    assert shape == (len(outs), 30) and rows == outs and idx == list(range(len(outs)))
+    # over the limit: a seeded sample whose rows and shape depend on the row count and the
+    # width only, not on what the rows hold; the files stay within the limit
+    limit = 4096 + 40 * (4 * 30 + 8)
+    bench.dump_outputs(str(tmp_path / "s1"), outs, width=30, limit=limit)
+    bench.dump_outputs(str(tmp_path / "s2"), ["x"] * len(outs), width=30, limit=limit)
+    for d in ("s1", "s2"):
+        assert sum(f.stat().st_size for f in (tmp_path / d).iterdir()) <= limit
+    shape, rows, idx = read(tmp_path / "s1")
+    assert shape == (40, 30) and idx == sorted(idx) and rows == [outs[i] for i in idx]
+    assert read(tmp_path / "s2")[::2] == (shape, idx)
+    # the width bounds every result the job can return: max_new_tokens tokens of the vocabulary
+    v = VB.build_vocab("qwen3", 1024, seed=0)
+    assert bench.dump_width(v, 24) == 24 * max(len(b) for b in v.token_bytes)
 
 
 def test_host_helpers():

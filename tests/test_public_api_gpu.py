@@ -26,9 +26,9 @@ class FreeSentiment(BaseModel):       # README.md:45-46 verbatim: a free string
 OPTS = dict(kv_pages=512, max_slots=8, max_prefill_tokens=512)
 
 
-def test_readme_flow_through_the_module_level_api():
+def test_readme_flow_through_the_module_level_api(tmp_path):
     import sutro_b200 as so
-    client = so.configure(engine_options=OPTS, verbose=False, cache_dir="/tmp/sb200-test-cache")
+    client = so.configure(engine_options=OPTS, verbose=False, cache_dir=str(tmp_path))
     df = pd.DataFrame({"review": synth.README_REVIEWS, "id": [7, 8, 9]})
     job_id = so.infer(df, column="review", model="tiny-qwen3",
                       system_prompt=synth.README_SYSTEM_PROMPT, output_schema=Sentiment)
@@ -67,10 +67,10 @@ def test_readme_flow_through_the_module_level_api():
     assert ok >= 1
 
 
-def test_templates_run_on_the_real_engine():
+def test_templates_run_on_the_real_engine(tmp_path):
     """classify / score / embed (sutro/templates/*.py call infer + await_job_completion)."""
     import sutro_b200 as so
-    so.configure(engine_options=OPTS, verbose=False, cache_dir="/tmp/sb200-test-cache")
+    so.configure(engine_options=OPTS, verbose=False, cache_dir=str(tmp_path))
     df = pd.DataFrame({"text": synth.product_reviews(6, seed=1)})
     cls = so.classify(df, ["good", "bad", "mixed"], model="tiny-qwen3", column="text")
     assert len(cls) == 6 and set(cls["inference_result"]) <= {"good", "bad", "mixed"}
@@ -81,11 +81,11 @@ def test_templates_run_on_the_real_engine():
     assert vecs.shape[0] == 6 and np.allclose(np.linalg.norm(vecs, axis=1), 1.0, atol=1e-3)
 
 
-def test_thinking_model_outputs_content_and_reasoning():
+def test_thinking_model_outputs_content_and_reasoning(tmp_path):
     """"<model>-thinking": reasoning first (capped), then the schema-constrained answer; the
     job reports {"content", "reasoning_content"} (sutro/sdk.py:1155-1164, common.py:28-32)."""
     import sutro_b200 as so
-    so.configure(engine_options=OPTS, verbose=False, cache_dir="/tmp/sb200-test-cache")
+    so.configure(engine_options=OPTS, verbose=False, cache_dir=str(tmp_path))
     rows = synth.README_REVIEWS + synth.product_reviews(5, seed=8)
     job = so.infer(rows, model="tiny-qwen3-thinking", system_prompt=synth.README_SYSTEM_PROMPT,
                    output_schema=Sentiment, sampling_params={"max_thinking_chars": 24},

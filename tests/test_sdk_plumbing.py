@@ -4,6 +4,8 @@ shaping follow the reference (sutro/common.py:72-163, sutro/sdk.py:186-193, :406
 these tests are about the host logic only."""
 import inspect
 import json
+import os
+import tempfile
 
 import numpy as np
 import pandas as pd
@@ -14,6 +16,12 @@ import sutro_b200 as so
 from sutro_b200 import common, interfaces
 from sutro_b200.engine import GenerationResult, rows_to_blob, blob_to_rows
 from sutro_b200.sdk import Sutro
+
+
+# the clients' results cache: private to this run (a fixed path under /tmp may belong to
+# another user of the machine)
+_CACHE = tempfile.TemporaryDirectory(prefix="sb200-test-cache-")
+CACHE = _CACHE.name
 
 
 class Sentiment(BaseModel):
@@ -32,7 +40,7 @@ class StubEngine:
 
 
 def client(as_json=True):
-    c = Sutro(verbose=False, cache_dir="/tmp/sb200-test-cache")
+    c = Sutro(verbose=False, cache_dir=CACHE)
     c.register_engine("qwen-3-4b", StubEngine(as_json))
     return c
 
@@ -147,7 +155,7 @@ def test_sampling_params_are_mapped_and_unknown_keys_rejected():
 
 
 def test_cumulative_logprobs_column():
-    c = Sutro(verbose=False, cache_dir="/tmp/sb200-test-cache")
+    c = Sutro(verbose=False, cache_dir=CACHE)
 
     class E:
         def generate(self, rows, **kw):
@@ -216,7 +224,7 @@ def test_template_signatures_match_reference():
 
 
 def test_classify_constrains_to_the_label_set():
-    c = Sutro(verbose=False, cache_dir="/tmp/sb200-test-cache")
+    c = Sutro(verbose=False, cache_dir=CACHE)
     eng = SchemaEcho()
     c.register_engine("m", eng)
     df = pd.DataFrame({"t": ["a", "b", "c"]})
@@ -232,7 +240,7 @@ def test_classify_constrains_to_the_label_set():
 
 
 def test_score_appends_bounded_integer_column():
-    c = Sutro(verbose=False, cache_dir="/tmp/sb200-test-cache")
+    c = Sutro(verbose=False, cache_dir=CACHE)
     eng = SchemaEcho()
     c.register_engine("m", eng)
     df = pd.DataFrame({"t": ["a", "b", "c"]})
@@ -247,7 +255,7 @@ def test_score_appends_bounded_integer_column():
 
 
 def test_embed_returns_vector_column():
-    c = Sutro(verbose=False, cache_dir="/tmp/sb200-test-cache")
+    c = Sutro(verbose=False, cache_dir=CACHE)
 
     class Emb:
         def generate(self, rows, **kw):
@@ -258,13 +266,13 @@ def test_embed_returns_vector_column():
     assert out["inference_result"][1].tolist() == [0, 1, 0, 0]
     import pyarrow.parquet as pq
     jid = c.list_jobs()[-1]["job_id"]
-    t = pq.read_table(f"/tmp/sb200-test-cache/{jid}.snappy.parquet")
+    t = pq.read_table(os.path.join(CACHE, f"{jid}.snappy.parquet"))
     assert t.column("inference_result").to_pylist()[1] == [0.0, 1.0, 0.0, 0.0]
     assert c.get_job_embeddings(jid).shape == (2, 4)
 
 
 def test_rank_returns_permutations_and_prints_elo(capsys):
-    c = Sutro(verbose=False, cache_dir="/tmp/sb200-test-cache")
+    c = Sutro(verbose=False, cache_dir=CACHE)
     eng = SchemaEcho()
     c.register_engine("m", eng)
     assert list(inspect.signature(Sutro.rank).parameters) == [
@@ -323,7 +331,7 @@ def test_rank_schemas_compile_to_permutation_dfas():
 
 
 def test_confidence_score_column_for_schema_jobs():
-    c = Sutro(verbose=False, cache_dir="/tmp/sb200-test-cache")
+    c = Sutro(verbose=False, cache_dir=CACHE)
 
     class E:
         def generate(self, rows, **kw):
@@ -344,7 +352,7 @@ def test_confidence_score_column_for_schema_jobs():
 
 def test_progress_records_have_the_reference_stream_shape():     # sutro/sdk.py:331-358
     seen = []
-    c = Sutro(verbose=False, cache_dir="/tmp/sb200-test-cache", on_progress=seen.append)
+    c = Sutro(verbose=False, cache_dir=CACHE, on_progress=seen.append)
 
     class E:
         def generate(self, rows, progress=None, **kw):
@@ -427,7 +435,7 @@ class _CutEngine(StubEngine):
 
 
 def test_one_unparsable_row_does_not_disable_json_unpacking():
-    c = Sutro(verbose=False, cache_dir="/tmp/sb200-test-cache")
+    c = Sutro(verbose=False, cache_dir=CACHE)
     c.register_engine("qwen-3-4b", _CutEngine())
     job = c.infer(["a", "b", "c"], model="qwen-3-4b", output_schema=Sentiment, stay_attached=False)
     df = c.get_job_results(job)
@@ -446,7 +454,7 @@ def test_default_output_budget_comes_from_the_schema():
 
         def compile_schema(self, schema, limits=None):
             return compile_schema(schema, limits)
-    c = Sutro(verbose=False, cache_dir="/tmp/sb200-test-cache")
+    c = Sutro(verbose=False, cache_dir=CACHE)
     eng = Eng()
     c.register_engine("qwen-3-4b", eng)
     enum_schema = {"type": "object", "properties": {"sentiment": {"type": "string", "enum": [
@@ -480,7 +488,7 @@ def test_files_and_frame_columns_travel_as_arrow(tmp_path):
             n = len(rows)
             return GenerationResult([f"o{i}" for i in range(n)], None, None,
                                     {"input_tokens": 1, "output_tokens": 1})
-    c = Sutro(verbose=False, cache_dir="/tmp/sb200-test-cache")
+    c = Sutro(verbose=False, cache_dir=CACHE)
     eng = ArrowEngine(as_json=False)
     c.register_engine("qwen-3-4b", eng)
     df = pd.DataFrame({"t": ["a", None, "c"], "n": [1, 2, 3]})
@@ -517,7 +525,7 @@ def test_thinking_models_report_content_and_reasoning():
             outs = [f"row {i} looks fine\n</think>\n\n" + json.dumps({"sentiment": f"s{i}"})
                     for i in range(len(rows))]
             return GenerationResult(outs, None, None, {"input_tokens": 1, "output_tokens": 1})
-    c = Sutro(verbose=False, cache_dir="/tmp/sb200-test-cache")
+    c = Sutro(verbose=False, cache_dir=CACHE)
     eng = ThinkEngine()
     c.register_engine("qwen-3-4b", eng)
     job = c.infer(["a", "b"], model="qwen-3-4b-thinking", output_schema=Sentiment,
