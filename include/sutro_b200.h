@@ -74,6 +74,10 @@ int sb200_rope_kv_write(void* qkv, const void* q_norm_w, const void* k_norm_w, c
                         const int32_t* page_table, int max_pages, void* kv_layer, int T, int hq,
                         int hkv, float eps, void* stream);
 
+/* Attention entry points (K2, K3): head_dim 128; hq must be a multiple of hkv with a GQA
+ * group hq/hkv of 1, 2, 4, 5 or 8.  Any other group returns -1 and sb200_last_error() names
+ * it ("unsupported GQA group size"). */
+
 /* K2: paged-KV decode attention, one query token per sequence. */
 int sb200_attn_decode(const void* qkv, void* out, const void* kv_layer, const int32_t* page_table,
                       int max_pages, const int32_t* row_slot, const int32_t* ctx_len, int B, int hq,
@@ -87,6 +91,7 @@ int sb200_attn_prefill(const void* qkv, void* out, const void* kv_layer, const i
                        int max_pages, const int32_t* work, int n_work, const int32_t* seq_slot,
                        const int32_t* seq_q_start, const int32_t* seq_q_len,
                        const int32_t* seq_past, int hq, int hkv, float scale, void* stream);
+/* tokens per prefill work item (q tile): 128 / (hq/hkv), e.g. 25 for group 5 */
 int sb200_attn_prefill_q_tile(int hq, int hkv);
 
 /* K3 on tcgen05 tensor cores (the engine's prefill path): causal varlen attention over DENSE

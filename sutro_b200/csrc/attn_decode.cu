@@ -416,6 +416,9 @@ int attn_decode(const void* qkv, void* out, const void* kv_layer, const int32_t*
     case 4:
       return launch<4>(qkv, out, kv_layer, page_table, max_pages, row_slot, ctx_len, B, hq, hkv,
                        scale, stream);
+    case 5:
+      return launch<5>(qkv, out, kv_layer, page_table, max_pages, row_slot, ctx_len, B, hq, hkv,
+                       scale, stream);
     case 8:
       return launch<8>(qkv, out, kv_layer, page_table, max_pages, row_slot, ctx_len, B, hq, hkv,
                        scale, stream);

@@ -4,9 +4,11 @@
 // new tokens attend to [cached prefix | themselves] through one code path; a
 // shared system-prompt prefix is just a run of shared page ids.
 //
-// Work decomposition: CTA = (q tile, kv head) of one sequence.  The CTA has 8
-// warps = G query heads x (QT/16) token sub-tiles, QT = 128/G, so all heads of
-// a GQA group reuse each K/V page loaded into shared memory.  Pages stream
+// Work decomposition: CTA = (q tile, kv head) of one sequence.  The CTA has
+// G query heads x ceil(QT/16) token sub-tiles warps, QT = 128/G (8 warps for
+// G = 1, 2, 4, 8; 10 for G = 5, whose 25-token tile ends inside the second
+// sub-tile), so all heads of a GQA group reuse each K/V page loaded into shared
+// memory.  Pages stream
 // through a 3-stage cp.async.bulk ring of 32-token super-tiles (two flat 8 KiB
 // copies of pre-swizzled tiles per stage, see kernels.h) so that one barrier
 // round and one softmax rescale cover 32 KV tokens; math is FlashAttention-2
@@ -20,14 +22,16 @@ namespace sb {
 
 namespace {
 
-constexpr int kPfWarps = 8;
 constexpr int kPfStages = 3;                    // ring of 32-token super-tiles (2 pages)
 constexpr int kPfStageBytes = 4 * kTileBytes;   // K0 | V0 | K1 | V1
 constexpr int kPfSmem = kPfStages * kPfStageBytes + 1024;
 constexpr int kPfMaxPages = 1024;               // 16 k tokens of context per sequence
 
+// warps per CTA: G heads x ceil(QT/16) sub-tiles
+constexpr int pf_warps(int G) { return G * ((128 / G + 15) / 16); }
+
 template <int G>
-__global__ void __launch_bounds__(kPfWarps * 32, 2)
+__global__ void __launch_bounds__(pf_warps(G) * 32, pf_warps(G) == 8 ? 2 : 1)
 attn_prefill_kernel(const __nv_bfloat16* __restrict__ qkv, __nv_bfloat16* __restrict__ out,
                     const __nv_bfloat16* __restrict__ kv_layer,
                     const int32_t* __restrict__ page_table, int max_pages,
@@ -35,6 +39,7 @@ attn_prefill_kernel(const __nv_bfloat16* __restrict__ qkv, __nv_bfloat16* __rest
                     const int32_t* __restrict__ seq_q_start, const int32_t* __restrict__ seq_q_len,
                     const int32_t* __restrict__ seq_past, int hq, int hkv, float scale_log2) {
   constexpr int QT = 128 / G;  // query tokens per CTA
+  constexpr int kWarps = pf_warps(G);
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>(
       (reinterpret_cast<uintptr_t>(smem_raw) + 127) & ~static_cast<uintptr_t>(127));
@@ -58,18 +63,22 @@ attn_prefill_kernel(const __nv_bfloat16* __restrict__ qkv, __nv_bfloat16* __rest
   const int sub = warp / G;                   // 16-token sub-tile of this warp
   const int q0 = qt0 + sub * 16;              // first query token (within the sequence's new tokens)
   const int cta_q_end = min(qt0 + QT, q_len);  // exclusive
+  // Tokens of this warp at or past q_end are not its to compute.  With QT a multiple of 16
+  // no sub-tile crosses the tile's end, so that is the sequence's end; otherwise (G = 5) the
+  // last sub-tile would also cover the first tokens of the next tile.
+  const int q_end = QT % 16 == 0 ? q_len : cta_q_end;
   const int last_kv_pos = past + cta_q_end - 1;
   const int n_pages = last_kv_pos / kPageTokens + 1;
   const int n_super = (n_pages + 1) >> 1;      // 32-token super-tiles
-  const int warp_last_pos = past + min(q0 + 16, q_len) - 1;  // causal horizon of this warp
-  const bool warp_active = q0 < q_len;
+  const int warp_last_pos = past + min(q0 + 16, q_end) - 1;  // causal horizon of this warp
+  const bool warp_active = q0 < q_end;
 
   if (threadIdx.x == 0) {
 #pragma unroll
     for (int s = 0; s < kPfStages; ++s) mbar_init(smem_u32(&full_bar[s]), 1);
     fence_mbar_init();
   }
-  for (int i = threadIdx.x; i < n_pages; i += kPfWarps * 32) s_pt[i] = pt[i];
+  for (int i = threadIdx.x; i < n_pages; i += kWarps * 32) s_pt[i] = pt[i];
   __syncthreads();
 
   // one super-tile = up to two pages, each one flat 8 KiB copy (K tile + V tile)
@@ -101,7 +110,7 @@ attn_prefill_kernel(const __nv_bfloat16* __restrict__ qkv, __nv_bfloat16* __rest
     const __nv_bfloat16* p0 =
         qkv + static_cast<size_t>(q_start + t0) * ldq + head * kHeadDim + 2 * (lane & 3);
     const __nv_bfloat16* p1 = p0 + static_cast<size_t>(8) * ldq;
-    const bool v0 = t0 < q_len, v1 = t1 < q_len;
+    const bool v0 = t0 < q_end, v1 = t1 < q_end;
 #pragma unroll
     for (int kk = 0; kk < 8; ++kk) {
       qa[kk][0] = v0 ? *reinterpret_cast<const uint32_t*>(p0 + kk * 16) : 0u;
@@ -227,7 +236,7 @@ attn_prefill_kernel(const __nv_bfloat16* __restrict__ qkv, __nv_bfloat16* __rest
 #pragma unroll
     for (int h = 0; h < 2; ++h) {
       const int t = q0 + r0 + 8 * h;
-      if (t >= q_len) continue;
+      if (t >= q_end) continue;
       const float inv = 1.0f / l_run[h];
       __nv_bfloat16* op = out + static_cast<size_t>(q_start + t) * hq * kHeadDim +
                           head * kHeadDim + 2 * (lane & 3);
@@ -248,7 +257,7 @@ int launch(const void* qkv, void* out, const void* kv_layer, const int32_t* page
   auto kern = attn_prefill_kernel<G>;
   SB_SET_MAX_SMEM(kern, kPfSmem);
   dim3 grid(n_work, hkv);
-  kern<<<grid, kPfWarps * 32, kPfSmem, stream>>>(
+  kern<<<grid, pf_warps(G) * 32, kPfSmem, stream>>>(
       static_cast<const __nv_bfloat16*>(qkv), static_cast<__nv_bfloat16*>(out),
       static_cast<const __nv_bfloat16*>(kv_layer), page_table, max_pages, work, seq_slot,
       seq_q_start, seq_q_len, seq_past, hq, hkv, scale * 1.4426950408889634f);
@@ -281,6 +290,7 @@ int attn_prefill(const void* qkv, void* out, const void* kv_layer, const int32_t
     case 1: SB_PF(1);
     case 2: SB_PF(2);
     case 4: SB_PF(4);
+    case 5: SB_PF(5);
     case 8: SB_PF(8);
     default:
       set_last_error("attn_prefill: unsupported GQA group size %d", hq / hkv);

@@ -12,7 +12,9 @@
 // Work item = (sequence, kv head, q tile).  A q tile packs QT = 128/G consecutive tokens x
 // the G query heads of the kv head into the 128 rows of one UMMA M tile (row = token*G +
 // head), so K/V are read once per GQA group and the causal frontier advances in QT-token
-// steps.  KV is consumed in blocks of up to 128 tokens: first the prefix blocks, then the
+// steps.  For G = 5 (QT = 25) the tile fills 125 rows; rows 125..127 are padding: their Q
+// rows are zero, their causal limit is the tile's last token and they never write output.
+// KV is consumed in blocks of up to 128 tokens: first the prefix blocks, then the
 // row's own blocks up to the tile's diagonal; the MMA N (and the PV K extent) is the valid
 // token count rounded up to 16, so short sequences do not pay for padding.
 //
@@ -48,6 +50,21 @@ constexpr int kBoxBytes = kBoxRows * 128;    // 4 KiB
 constexpr int kTcBarBytes = 256;
 constexpr int kTcSmem = 7 * kTileBytes2 + kTcBarBytes + 1024;  // Q[2] K[2] V[2] P + barriers + align
 constexpr float kRescaleThreshold = 8.0f;    // log2 units: P stays <= 2^8 before a forced rescale
+
+// Q tile of a GQA group of G heads: QT = 128/G tokens x G heads, loaded as two d-halves of
+// one TMA box {64, G, QT}.  The box (tc_maps) and the Q_FULL transaction count are both
+// derived from here: a count that differs from the bytes TMA delivers never completes.
+constexpr int tc_q_tokens(int G) { return 128 / G; }
+constexpr int tc_q_rows(int G) { return tc_q_tokens(G) * G; }  // tile rows TMA fills
+constexpr int tc_q_bytes(int G) { return 2 * tc_q_rows(G) * 64 * 2; }
+template <int G>
+constexpr bool tc_q_bytes_ok() {
+  static_assert(tc_q_rows(G) <= 128 && tc_q_rows(G) > 120, "the q tile must nearly fill M = 128");
+  static_assert(tc_q_bytes(G) == 2 * (kHalfBytes / 128) * tc_q_rows(G), "Q bytes != box bytes");
+  static_assert(tc_q_bytes(G) % 16 == 0 && tc_q_bytes(G) <= kTileBytes2, "Q box overflows");
+  static_assert(tc_q_rows(G) < 128 || tc_q_bytes(G) == kTileBytes2, "full tile != 32 KiB");
+  return true;
+}
 
 struct TcGeom {
   int q_start, q_len, past, qt0, kvh;
@@ -124,6 +141,9 @@ attn_prefill_tc_kernel(const __grid_constant__ CUtensorMap tm_q,    // 3-D (d, h
                        const int32_t* __restrict__ seq_q_len, const int32_t* __restrict__ seq_past,
                        int hq, int hkv, int layer, float scale_log2) {
   constexpr int QT = 128 / G;
+  constexpr int kQRows = tc_q_rows(G);
+  constexpr bool kPad = kQRows < 128;  // G = 5: tile rows kQRows..127 are padding
+  static_assert(QT == tc_q_tokens(G) && tc_q_bytes_ok<G>(), "q tile geometry");
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>(
       (reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~static_cast<uintptr_t>(1023));
@@ -158,6 +178,17 @@ attn_prefill_tc_kernel(const __grid_constant__ CUtensorMap tm_q,    // 3-D (d, h
     tmem_alloc(smem_u32(tmem_slot), 512);
     tmem_relinquish();
   }
+  if constexpr (kPad) {
+    // TMA never writes the padding rows of the Q buffers: zero them once (both buffers, both
+    // d-halves), so that their scores are exactly 0 and independent of what smem held before
+    constexpr int kPadChunks = (128 - kQRows) * 128 / 16;  // 16-byte stores per d-half
+    for (int i = threadIdx.x; i < 4 * kPadChunks; i += kTcThreads) {
+      const int half = i / kPadChunks;  // (Q buffer, d-half) pair: 2 x 2
+      const uint32_t a = s_q + half * kHalfBytes + kQRows * 128 + (i - half * kPadChunks) * 16;
+      asm volatile("st.shared.v4.u32 [%0], {%1,%1,%1,%1};" ::"r"(a), "r"(0u) : "memory");
+    }
+    fence_proxy_async_smem();  // generic stores -> visible to the UMMA (async proxy)
+  }
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
@@ -180,7 +211,7 @@ attn_prefill_tc_kernel(const __grid_constant__ CUtensorMap tm_q,    // 3-D (d, h
         if (!v_flow) {
           const uint32_t qb = n & 1;
           mbar_wait(bar(Q_EMPTY + qb), ((n >> 1) & 1) ^ 1);
-          mbar_arrive_expect_tx(bar(Q_FULL + qb), kTileBytes2);
+          mbar_arrive_expect_tx(bar(Q_FULL + qb), tc_q_bytes(G));
           const uint32_t qd = s_q + qb * kTileBytes2;
           tma_load_3d(qd, &tm_q, bar(Q_FULL + qb), 0, ge.kvh * G, ge.q_start + ge.qt0);
           tma_load_3d(qd + kHalfBytes, &tm_q, bar(Q_FULL + qb), 64, ge.kvh * G,
@@ -296,6 +327,11 @@ attn_prefill_tc_kernel(const __grid_constant__ CUtensorMap tm_q,    // 3-D (d, h
     const int r = warp * 32 + lane;       // tile row == TMEM lane
     const int t_in = r / G;               // token within the q tile
     const int h_in = r - t_in * G;        // query head within the GQA group
+    // A padding row (kPad) takes the causal limit of the tile's last token: the largest in the
+    // tile, so limits still grow with the lane (vmin below), and only columns that a real row
+    // also reads.  It never writes output.
+    const bool row_real = !kPad || r < kQRows;
+    const int t_lim = kPad ? min(t_in, QT - 1) : t_in;
     const uint32_t lane_sel = static_cast<uint32_t>(warp * 32) << 16;
     const uint32_t p_row = s_p + r * 128;
     const int sw = r & 7;
@@ -344,7 +380,7 @@ attn_prefill_tc_kernel(const __grid_constant__ CUtensorMap tm_q,    // 3-D (d, h
     };
     for (int item = blockIdx.x; item < n_items_total; item += gridDim.x, ++n) {
       const TcGeom ge = tc_geom<G>(item, hkv, items, seq_q_start, seq_q_len, seq_past);
-      const int q_own = ge.qt0 + t_in;    // index of this row's token among the own tokens
+      const int q_own = ge.qt0 + t_lim;   // index of this row's token among the own tokens
       const uint32_t ob = n & 1;
       for (int b = 0; b < ge.n_blocks; ++b, ++g) {
         bool is_pre;
@@ -478,7 +514,7 @@ attn_prefill_tc_kernel(const __grid_constant__ CUtensorMap tm_q,    // 3-D (d, h
           ep_ob = ob;
           ep_par = (n >> 1) & 1;
           ep_inv = 1.0f / l_run;
-          ep_row_ok = q_own < ge.q_len;
+          ep_row_ok = row_real && q_own < ge.q_len;
           ep_dst = out + static_cast<size_t>(ge.q_start + q_own) * (hq * kHeadDim) +
                    (ge.kvh * G + h_in) * kHeadDim;
         }
@@ -535,7 +571,8 @@ int tc_maps(const TcKey& key, TcMaps* out) {
     const uint64_t dims[3] = {static_cast<uint64_t>(kHeadDim), static_cast<uint64_t>(key.hq),
                               static_cast<uint64_t>(key.t_rows)};
     const uint64_t strides[2] = {kHeadDim * 2ull, ldq * 2ull};
-    const uint32_t box[3] = {64u, static_cast<uint32_t>(G), static_cast<uint32_t>(128 / G)};
+    const uint32_t box[3] = {64u, static_cast<uint32_t>(G),
+                             static_cast<uint32_t>(tc_q_tokens(G))};
     if (encode_tmap_bf16(&m.q, key.qkv, 3, dims, strides, box)) return -1;
   }
   {
@@ -609,6 +646,7 @@ int attn_prefill_dense(const void* qkv, int t_rows, void* out, const void* prefi
     case 1: SB_TC(1);
     case 2: SB_TC(2);
     case 4: SB_TC(4);
+    case 5: SB_TC(5);
     case 8: SB_TC(8);
     default:
       set_last_error("attn_prefill_dense: unsupported GQA group size %d", hq / hkv);

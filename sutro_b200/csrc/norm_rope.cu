@@ -241,6 +241,8 @@ int rmsnorm(const void* x, const void* w, void* out, int rows, int d, float eps,
     rmsnorm_kernel<10><<<grid, block, 0, stream>>>(xp, wp, op, rows, d, eps);
   else if (nvec <= 32 * 16)
     rmsnorm_kernel<16><<<grid, block, 0, stream>>>(xp, wp, op, rows, d, eps);
+  else if (nvec <= 32 * 20)  // d <= 5120 (Qwen3-14B / 32B)
+    rmsnorm_kernel<20><<<grid, block, 0, stream>>>(xp, wp, op, rows, d, eps);
   else
     rmsnorm_kernel<0><<<grid, block, 0, stream>>>(xp, wp, op, rows, d, eps);
   SB_CUDA_CHECK(cudaGetLastError());

@@ -87,6 +87,11 @@ QWEN3_0_6B = _reg(ModelSpec("qwen-3-0.6b", "qwen3", 28, 1024, 16, 8, 3072, 15193
 QWEN3_EMB_0_6B = _reg(replace(QWEN3_0_6B, name="qwen-3-embedding-0.6b", embedding_model=True))
 QWEN3_4B = _reg(ModelSpec("qwen-3-4b", "qwen3", 36, 2560, 32, 8, 9728, 151936, True, 1e-6, 1e6,
                           True))
+# GQA group 5 (40 q / 8 kv heads): the attention kernels' only non-power-of-two group
+QWEN3_14B = _reg(ModelSpec("qwen-3-14b", "qwen3", 40, 5120, 40, 8, 17408, 151936, False, 1e-6,
+                           1e6, True))
+QWEN3_32B = _reg(ModelSpec("qwen-3-32b", "qwen3", 64, 5120, 64, 8, 25600, 151936, False, 1e-6,
+                           1e6, True))
 LLAMA31_8B = _reg(ModelSpec("llama-3.1-8b", "llama", 32, 4096, 32, 8, 14336, 128256, False, 1e-5,
                             5e5, False, rope_scaling=_LLAMA31_SCALING))
 # BASELINE.json says "llama-3-8b"; the reference's ModelOptions lists llama-3.1-8b
@@ -99,6 +104,8 @@ TINY_QWEN3 = _reg(ModelSpec("tiny-qwen3", "qwen3", 2, 256, 4, 2, 512, 1024, True
                             max_position=512))
 TINY_QWEN3_G4 = _reg(ModelSpec("tiny-qwen3-g4", "qwen3", 3, 512, 8, 2, 768, 2048, True, 1e-6, 1e6,
                                True, max_position=1024))
+TINY_QWEN3_G5 = _reg(ModelSpec("tiny-qwen3-g5", "qwen3", 3, 512, 10, 2, 768, 2048, True, 1e-6,
+                               1e6, True, max_position=1024))
 TINY_LLAMA = _reg(ModelSpec("tiny-llama", "llama", 2, 256, 4, 2, 512, 1024, False, 1e-5, 5e5,
                             False, max_position=512, rope_scaling=_LLAMA31_SCALING))
 TINY_EMB = _reg(replace(TINY_QWEN3, name="tiny-qwen3-embedding", embedding_model=True))

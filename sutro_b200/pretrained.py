@@ -10,7 +10,7 @@ same engine serves the real model:
 What is read: `config.json` (architecture → ModelSpec), `tokenizer.json` (byte-level BPE
 vocabulary, merges, special tokens), `*.safetensors` (+ `model.safetensors.index.json` when
 sharded).  Supported architectures are the ones the kernels cover: Qwen3 and Llama-3 dense
-decoders with head_dim 128 and a GQA group of 1, 2, 4 or 8.
+decoders with head_dim 128 and a GQA group of 1, 2, 4, 5 or 8 (5: Qwen3-14B, 40 q / 8 kv heads).
 
 Token ids.  The GPU tokenizer starts from raw byte values, so the engine's id space has byte b
 at id b.  GPT-2-style vocabularies keep the 256 byte tokens at ids 0..255 in another order;
@@ -163,13 +163,18 @@ def spec_from_hf_config(cfg: Dict[str, Any], name: str, max_position: int = 4096
     if head_dim != MS.HEAD_DIM:
         raise ValueError(f"head_dim {head_dim} is not supported (kernels are built for "
                          f"{MS.HEAD_DIM})")
-    if hq % hkv or hq // hkv not in (1, 2, 4, 8):
-        raise ValueError(f"GQA group {hq}/{hkv} is not supported (1, 2, 4 or 8)")
+    if hq % hkv or hq // hkv not in (1, 2, 4, 5, 8):
+        raise ValueError(f"GQA group {hq}/{hkv} is not supported (1, 2, 4, 5 or 8)")
     if cfg.get("attention_bias") or cfg.get("mlp_bias"):
         raise ValueError("projection biases are not supported")
     if cfg.get("sliding_window") and cfg.get("use_sliding_window"):
         raise ValueError("sliding-window attention is not supported")
+    # transformers >= 5 writes rope_theta (and any scaling) under rope_parameters
+    rope_params = cfg.get("rope_parameters") or {}
+    theta = cfg.get("rope_theta") or rope_params.get("rope_theta", 1e4)
     scaling = cfg.get("rope_scaling")
+    if scaling is None and rope_params.get("rope_type", "default") != "default":
+        scaling = rope_params
     if scaling is not None:
         kind = scaling.get("rope_type", scaling.get("type"))
         if kind != "llama3":
@@ -181,7 +186,7 @@ def spec_from_hf_config(cfg: Dict[str, Any], name: str, max_position: int = 4096
         n_layers=int(cfg["num_hidden_layers"]), d_model=d_model, n_q_heads=hq, n_kv_heads=hkv,
         d_ff=int(cfg["intermediate_size"]), vocab_size=int(cfg["vocab_size"]),
         tied_embeddings=bool(cfg.get("tie_word_embeddings", False)),
-        rms_eps=float(cfg.get("rms_norm_eps", 1e-6)), rope_theta=float(cfg.get("rope_theta", 1e4)),
+        rms_eps=float(cfg.get("rms_norm_eps", 1e-6)), rope_theta=float(theta),
         qk_norm=(mt == "qwen3"),
         max_position=min(int(cfg.get("max_position_embeddings", max_position)), max_position),
         rope_scaling=scaling, embedding_model=embedding_model)
